@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (ours)
     python bench.py --impl reference --gpus N --steps K --warmup W   (the reference's CPU encoder)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR    (also write the files of the last step)
 
 A "step" is one pass of the hot path over one batch of synthetic images.
 Default workload = BASELINE.json configs[1]: a batch of 256 synthetic
@@ -64,7 +65,11 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-parity-gate", action="store_true", help="development only: skip the untimed byte comparison with the reference")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the JPEG files of rank 0's last step to DIR as .npy (see dump_outputs)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     w = WORKLOADS[a.workload]
     a.custom = any(v is not None for v in (a.batch, a.width, a.height, a.switches))
     for k in ("batch", "width", "height", "switches"):
@@ -367,6 +372,23 @@ def parity_gate(outputs, images, switches, who):
     return {"checked_images": len(images), "against": "oracle/_ref (unmodified reference)" if use_ref else "oracle port", "identical": True}
 
 
+def dump_outputs(path, files, budget=64 * 10**6):
+    """--dump-outputs: the JPEG files one step returned, as float32 byte values, so that two builds can be compared
+    output for output.  jpeg_sizes.npy holds every file's length in bytes; jpeg_bytes.npy the files of a seeded sample
+    of the batch, concatenated in image order; jpeg_images.npy the indices of those images.  The sample takes whole
+    files in a fixed random order while the three arrays stay within `budget` bytes (all files when they fit)."""
+    os.makedirs(path, exist_ok=True)
+    room = (budget - 3 * 4096 - 16 * len(files)) // 4          # npy headers, sizes + indices as float64
+    pick = []
+    for i in np.random.default_rng(0).permutation(len(files)):
+        if len(files[i]) <= room:
+            pick.append(int(i)); room -= len(files[i])
+    pick.sort()
+    np.save(os.path.join(path, "jpeg_sizes.npy"), np.array([len(f) for f in files], dtype=np.float64))
+    np.save(os.path.join(path, "jpeg_images.npy"), np.array(pick, dtype=np.float64))
+    np.save(os.path.join(path, "jpeg_bytes.npy"), np.frombuffer(b"".join(files[i] for i in pick), dtype=np.uint8).astype(np.float32))
+
+
 def measure(a, sw, enc, host, devbuf, base, rank, world, local, dev, stream, dist, torch):
     """One configuration (switch set) on the already staged batch: resident value, e2e, stage times, parity gate."""
     import mozjpeg_b200 as mj
@@ -430,6 +452,9 @@ def measure(a, sw, enc, host, devbuf, base, rank, world, local, dev, stream, dis
     else:
         step_e2e()                                     # the parity gate needs files
         jpeg_bytes = sum(enc.output_size(i) for i in range(B))
+    # the files of the last step (the resident steps encode the same pixels with the same parameters but leave their
+    # entropy-coded bytes in HBM; the end-to-end call is the one that returns files)
+    files = [enc.get_output(i) for i in range(B)] if a.dump_outputs and rank == 0 else None
 
     # ---- parity gate (untimed): first and last image of this rank's batch against the reference ----
     gate = None
@@ -437,7 +462,7 @@ def measure(a, sw, enc, host, devbuf, base, rank, world, local, dev, stream, dis
         idx = sorted({0, B - 1})
         gate = parity_gate([enc.get_output(i) for i in idx], [base[i % len(base)] for i in idx], sw, f"rank {rank}, {' '.join(sw)}")
     return {"ms_total": ms_total, "launches": launches, "stages": stages, "chunk": chunk, "clk": clk, "e2e_ms": e2e_ms,
-            "jpeg_bytes": jpeg_bytes, "gate": gate, "B": B}
+            "jpeg_bytes": jpeg_bytes, "gate": gate, "B": B, "files": files}
 
 
 def main():
@@ -500,6 +525,8 @@ def main():
         for q in a.sweep:
             sw = a.switches.replace("-quality 75", f"-quality {q}").split()
             runs[q] = measure(a, sw, enc, host, devbuf, base, rank, world, local, dev, stream, dist, torch)
+            if q != 75:
+                runs[q]["files"] = None                # the reported value is q75's
         r = runs[75]
     else:
         r = measure(a, a.switches.split(), enc, host, devbuf, base, rank, world, local, dev, stream, dist, torch)
@@ -576,6 +603,8 @@ def main():
         latency = {"ms": statistics.median(lat[1:]), "first_call_ms": lat[0], "bytes": len(data),
                    "what": "b200jpeg_start_compress + write_scanlines (all rows, pageable host memory) + finish_compress, one image, median of 4"}
 
+    if r["files"] is not None:
+        dump_outputs(a.dump_outputs, r["files"])
     if rank == 0:
         cfg = {"workload": workload_name(a), "images_per_gpu": B, "global_images": global_images,
                "l2": "inputs (%.1f GB per GPU) exceed the 126 MB L2" % (B * in_bytes / 1e9),

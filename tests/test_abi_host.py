@@ -66,18 +66,18 @@ def test_switch_semantics(built):
 
 
 def test_quant_tables_match_reference_dqt(built):
-    """Tables we derive == tables the reference writes into its DQT."""
+    """Tables we derive == tables the reference writes into its DQT (as its decoder reads them back, per component;
+    tests/golden/dqt_golden.json)."""
+    import json
     import mozjpeg_b200 as mj
-    from oracle import oracle as O
-    if not O.ref_available():
-        pytest.skip("oracle/_ref not built")
-    img = O.synth_image(1, 32, 32)
-    for sw in (["-revert"], ["-baseline", "-quality", "75"], ["-baseline", "-quality", "33"], ["-baseline", "-quality", "97"],
-               ["-baseline", "-quant-table", "5", "-quality", "60"], ["-revert", "-quality", "5"]):
+    from common import GOLD
+    cases = json.load(open(os.path.join(GOLD, "dqt_golden.json")))["cases"]
+    assert len(cases) == 6
+    for c in cases:
+        sw, qt = c["switches"], c["qt"]
         p = mj.params_from_switches(sw, 32, 32)
-        qt = O.ref_read_coefs(O.ref_encode(img, sw))["qt"]
         for ci in range(3):
-            assert list(p.quant_tbl[p.comp_info[ci].quant_tbl_no]) == qt[ci].tolist(), (sw, ci)
+            assert list(p.quant_tbl[p.comp_info[ci].quant_tbl_no]) == qt[ci], (sw, ci)
 
 
 def test_validation_errors(built):

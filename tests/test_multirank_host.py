@@ -42,16 +42,15 @@ def test_shards_and_max_reduction_over_gloo(built):
 
 
 def test_reference_arm_under_torchrun_prints_once(built):
+    """Where oracle/_ref is not built the arm runs the oracle port and must say so."""
     from oracle import oracle as O
-    if not O.ref_available():
-        import pytest
-        pytest.skip("oracle/_ref not built")
     r = _torchrun([os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "0", "--width", "64", "--height", "48"])
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [ln for ln in r.stdout.splitlines() if ln.startswith("{")]
     assert len(lines) == 1, r.stdout
     d = json.loads(lines[0])
-    assert d["impl"] == "reference" and d["n_gpus"] == 2 and d["e2e"]["h2d_bytes_per_step"] == 0 and d["cpu_baseline"]["kind"] == "reference"
+    assert d["impl"] == "reference" and d["n_gpus"] == 2 and d["e2e"]["h2d_bytes_per_step"] == 0
+    assert d["cpu_baseline"]["kind"] == ("reference" if O.ref_available() else "port")
 
 
 def _bench_module():
@@ -61,13 +60,20 @@ def _bench_module():
     return m
 
 
-def test_clock_sampler_window_and_fallback():
+def _no_nvidia_smi(*args, **kwargs):
+    raise FileNotFoundError("nvidia-smi")
+
+
+def test_clock_sampler_window_and_fallback(monkeypatch):
     """bench.py's `clocks` entry: the samples between the two marks are the ones reported (median SM clock, union of the
     throttle reasons), a timed region shorter than one sampling period falls back to warm-up + timed region and says so,
     and a box without NVML / nvidia-smi yields a null entry instead of an exception."""
     b = _bench_module()
-    c = b.ClockSampler(0)
-    c.start(); out = c.stop(0, None)                      # no GPU here: neither source comes up
+    with monkeypatch.context() as m:                      # neither source comes up, also where a GPU is present
+        m.setitem(sys.modules, "pynvml", None)
+        m.setattr(b.subprocess, "Popen", _no_nvidia_smi)
+        c = b.ClockSampler(0)
+        c.start(); out = c.stop(0, None)
     assert out["samples"] == 0 and out["sm_mhz"] is None
     c = b.ClockSampler(0); c.source = "nvml"
     c.samples = [(1500.0, 1965.0, ()), (1600.0, 1965.0, ())]                       # warm-up
@@ -81,3 +87,26 @@ def test_clock_sampler_window_and_fallback():
     c = b.ClockSampler(0); c.source = "nvml"; c.samples = [(1800.0, 1965.0, ())]
     out = c.stop(1, 1)                                    # nothing inside the marks
     assert out["samples"] == 1 and out["window"].startswith("warm-up")
+
+
+def test_dump_outputs_sample_and_budget(tmp_path):
+    """bench.py --dump-outputs: every file's size, whole files of a fixed sample within the byte budget, float32 bytes."""
+    import numpy as np
+    b = _bench_module()
+    rng = np.random.default_rng(1)
+    files = [rng.integers(0, 256, int(n), dtype=np.uint8).tobytes() for n in rng.integers(1000, 50000, 40)]
+    b.dump_outputs(str(tmp_path / "all"), files)                      # everything fits
+    sizes = np.load(tmp_path / "all" / "jpeg_sizes.npy"); images = np.load(tmp_path / "all" / "jpeg_images.npy")
+    data = np.load(tmp_path / "all" / "jpeg_bytes.npy")
+    assert sizes.dtype == np.float64 and images.dtype == np.float64 and data.dtype == np.float32
+    assert sizes.tolist() == [len(f) for f in files] and images.tolist() == list(range(40))
+    assert data.astype(np.uint8).tobytes() == b"".join(files)
+    budget = 300000
+    for run in ("a", "b"):
+        b.dump_outputs(str(tmp_path / run), files, budget)
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= budget
+    images = np.load(tmp_path / "a" / "jpeg_images.npy").astype(int).tolist()
+    assert 0 < len(images) < 40 and images == sorted(images)
+    assert np.load(tmp_path / "a" / "jpeg_bytes.npy").astype(np.uint8).tobytes() == b"".join(files[i] for i in images)
+    for f in ("jpeg_sizes.npy", "jpeg_images.npy", "jpeg_bytes.npy"):          # the same sample every time
+        assert (tmp_path / "a" / f).read_bytes() == (tmp_path / "b" / f).read_bytes()

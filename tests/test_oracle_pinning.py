@@ -3,8 +3,9 @@
 * against the reference's own golden vector (testimages/testimgint.jpg ==
   `cjpeg -revert -dct int testorig.ppm`, md5 in CMakeLists.txt:1391) and the
   md5s recorded from the unmodified reference by tools/make_golden.py;
-* live, byte for byte, against oracle/_ref when it is built (container and GPU
-  box both carry it; skipped otherwise).
+* against what the reference's library, its forward DCT and its cjpeg binary
+  made of seeded odd-shaped inputs and random switch sets, recorded by
+  tools/make_golden.py --checks.
 """
 import os
 
@@ -71,45 +72,40 @@ def test_oracle_full_size_recorded_reference(built, case):
 
 
 def test_oracle_live_vs_reference_random_shapes(built):
-    """Odd shapes x profiles, live against the compiled reference."""
+    """Odd shapes x profiles against the reference's bytes for them (tests/golden/random_shapes_golden.json)."""
+    import json
     import mozjpeg_b200 as mj
+    from common import GOLD
     from oracle import oracle as O
-    if not O.ref_available():
-        pytest.skip("oracle/_ref not built")
-    rng = np.random.default_rng(7)
-    sws = [["-baseline", "-quality", "70"], ["-fastcrush", "-quality", "80"], ["-revert", "-optimize"],
-           ["-baseline", "-quality", "75", "-sample", "2x1"], ["-baseline", "-quality", "75", "-sample", "1x2"]]
-    for _ in range(12):
-        w, h = int(rng.integers(1, 97)), int(rng.integers(1, 97))
-        img = O.synth_image(int(rng.integers(0, 1 << 30)), w, h)
-        for sw in sws:
-            p = mj.params_from_switches(sw, w, h)
-            assert O.oracle_encode(p, img).jpeg == O.ref_encode(img, sw), (w, h, sw)
+    cases = json.load(open(os.path.join(GOLD, "random_shapes_golden.json")))["cases"]
+    assert len(cases) == 60
+    for c in cases:
+        w, h, sw = c["width"], c["height"], c["switches"]
+        p = mj.params_from_switches(sw, w, h)
+        out = O.oracle_encode(p, O.synth_image(c["seed"], w, h)).jpeg
+        assert (len(out), md5(out)) == (c["size"], c["md5"]), (w, h, sw)
 
 
 def test_stage_oracles_vs_reference_internals(built):
-    """jpeg_fdct_islow of the reference library vs our restatement."""
+    """jpeg_fdct_islow of the reference library vs our restatement, on 200 random blocks (tests/golden/fdct_islow_golden.npz)."""
     import ctypes as C
+    from common import GOLD
     from oracle import oracle as O
-    if not O.ref_available():
-        pytest.skip("oracle/_ref not built")
-    rng = np.random.default_rng(3)
-    for _ in range(200):
-        blk = rng.integers(-128, 160, 64).astype(np.int32)
-        a = blk.copy(); b = blk.copy()
+    g = np.load(os.path.join(GOLD, "fdct_islow_golden.npz"))
+    assert g["input"].shape == (200, 64)
+    for blk, want in zip(g["input"], g["output"]):
+        a = blk.astype(np.int32)
         O.orc().orc_fdct_islow(a.ctypes.data_as(C.POINTER(C.c_int)))
-        O.ref().refshim_fdct_islow(b.ctypes.data_as(C.POINTER(C.c_int)))
-        assert (a == b).all()
+        assert (a == want).all()
 
 
 def test_random_switch_sets_live_against_reference_cjpeg(built):
     """tools/fuzz_vs_reference.py, a short run: random cjpeg switch sets (profiles, quality, sampling, restarts, DCT,
-    smoothing, tuning presets, lambda, DC weight) on random small images - reference binary vs mirror + oracle."""
+    smoothing, tuning presets, lambda, DC weight) on random small images - what the reference's cjpeg binary did with each
+    (accepted or refused, and its bytes; tests/golden/fuzz_golden.json) vs mirror + oracle."""
     import subprocess
     import sys
-    from common import ROOT
-    from oracle import oracle as O
-    if not (O.ref_available() and os.path.exists(os.path.join(O.REF_DIR, "cjpeg"))):
-        pytest.skip("oracle/_ref not built")
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "fuzz_vs_reference.py"), "2024", "60"], capture_output=True, text=True, timeout=900)
+    from common import GOLD, ROOT
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "fuzz_vs_reference.py"), "2024", "60",
+                        "--recorded", os.path.join(GOLD, "fuzz_golden.json")], capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-500:]

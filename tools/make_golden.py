@@ -169,7 +169,71 @@ FULLSIZE = [
     ([26, 3840, 2160, 12], ["-precision", "12", "-sample", "1x1", "-quality", "75", "-notrellis", "-noovershoot", "-baseline"]),   # configs[4]
     ([1000, 3840, 2160, 12], ["-precision", "12", "-sample", "1x1", "-quality", "75", "-notrellis", "-noovershoot", "-baseline"]),
     ([300, 3840, 2160], ["-quality", "75", "-sample", "2x2"]),                       # the library default (scan search) at 4K
+    ([301, 3840, 2160], ["-baseline", "-quality", "75", "-sample", "2x2"]),          # second image of test_full_size_4k_frame
 ]
+
+
+def reference_checks():
+    """--checks: fixtures of the checks against the reference's library and binaries: odd shapes x profiles, the forward DCT on
+    random blocks, the quantization tables of the reference's DQT, a recorded run of tools/fuzz_vs_reference.py, and
+    the coefficient-domain re-encode of odd source files (the sources, their coefficients and jpegtran's md5s)."""
+    import subprocess
+    import ctypes as C
+    from mozjpeg_b200.synth import synth_image12
+    # test_oracle_pinning: odd shapes x profiles
+    rng = np.random.default_rng(7)
+    sws = [["-baseline", "-quality", "70"], ["-fastcrush", "-quality", "80"], ["-revert", "-optimize"],
+           ["-baseline", "-quality", "75", "-sample", "2x1"], ["-baseline", "-quality", "75", "-sample", "1x2"]]
+    shapes = []
+    for _ in range(12):
+        w, h = int(rng.integers(1, 97)), int(rng.integers(1, 97))
+        seed = int(rng.integers(0, 1 << 30))
+        im = O.synth_image(seed, w, h)
+        for sw in sws:
+            a = O.ref_encode(im, sw)
+            shapes.append({"seed": seed, "width": w, "height": h, "switches": sw, "md5": hashlib.md5(a).hexdigest(), "size": len(a)})
+    json.dump({"generator": "tools/make_golden.py --checks", "cases": shapes}, open(os.path.join(GOLD, "random_shapes_golden.json"), "w"), indent=0)
+    # test_oracle_pinning: jpeg_fdct_islow of the reference library on random blocks
+    rng = np.random.default_rng(3)
+    blocks = rng.integers(-128, 160, (200, 64)).astype(np.int32)
+    out = blocks.copy()
+    for b in out:
+        O.ref().refshim_fdct_islow(b.ctypes.data_as(C.POINTER(C.c_int)))
+    np.savez_compressed(os.path.join(GOLD, "fdct_islow_golden.npz"), input=blocks, output=out)
+    # test_abi_host: the quantization tables the reference writes into its DQT
+    img = O.synth_image(1, 32, 32)
+    dqt = []
+    for sw in (["-revert"], ["-baseline", "-quality", "75"], ["-baseline", "-quality", "33"], ["-baseline", "-quality", "97"],
+               ["-baseline", "-quant-table", "5", "-quality", "60"], ["-revert", "-quality", "5"]):
+        dqt.append({"switches": sw, "qt": O.ref_read_coefs(O.ref_encode(img, sw))["qt"].tolist()})
+    json.dump({"generator": "tools/make_golden.py --checks", "cases": dqt}, open(os.path.join(GOLD, "dqt_golden.json"), "w"), indent=0)
+    # test_oracle_pinning: random cjpeg switch sets through the reference's cjpeg binary
+    subprocess.check_call([sys.executable, os.path.join(ROOT, "tools", "fuzz_vs_reference.py"), "2024", "60",
+                           "--record", os.path.join(GOLD, "fuzz_golden.json")])
+    # test_transcode: source files the encode fixture does not have (16-bit quantization tables, RGB colourspace,
+    # restart markers, gray with 2x2 sampling, 12-bit), their coefficients as the reference's decoder reads them, and
+    # what the reference's jpegtran makes of them
+    im = O.synth_image(3, 120, 72)
+    srcs = []
+    for esw in (["-revert", "-quality", "3"], ["-quality", "12", "-sample", "2x2"], ["-revert", "-rgb"], ["-revert", "-progressive", "-restart", "1"],
+                ["-revert", "-quality", "50", "-sample", "2x2", "-grayscale"]):      # a gray file with 2x2 sampling leaves jpegtran as 1x1
+        try:
+            srcs.append(O.ref_encode(im, esw))
+        except ValueError:
+            srcs.append(O._ref_cjpeg_pixels(im, esw))
+    srcs.append(O.ref_encode(synth_image12(4, 120, 72), ["-precision", "12", "-quality", "75", "-notrellis", "-noovershoot", "-baseline"]))
+    trans = ([], ["-revert"], ["-progressive"], ["-revert", "-optimize"])
+    arrays = {}
+    md5s, sizes = [], []
+    for k, src in enumerate(srcs):
+        arrays["src%d" % k] = np.frombuffer(src, dtype=np.uint8)
+        for ci, plane in enumerate(O.ref_read_coefs(src)["coefs"]):
+            arrays["coef%d_%d" % (k, ci)] = plane
+        outs = [O.ref_jpegtran(src, tsw) for tsw in trans]
+        md5s.append([hashlib.md5(a).hexdigest() for a in outs]); sizes.append([len(a) for a in outs])
+    np.savez_compressed(os.path.join(GOLD, "transcode_odd_golden.npz"), tran=np.array([" ".join(t) for t in trans]),
+                        md5=np.array(md5s), size=np.array(sizes), **arrays)
+    print("wrote the reference-check fixtures")
 
 
 def fullsize():
@@ -195,6 +259,8 @@ def fullsize():
 def main():
     if "--fullsize" in sys.argv:
         return fullsize()
+    if "--checks" in sys.argv:
+        return reference_checks()
     os.makedirs(GOLD, exist_ok=True)
     # cases already recorded are kept as they are unless --force is given (a full regeneration takes a while)
     have = {}
